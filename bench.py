@@ -32,6 +32,8 @@ Printed JSON (one line, rank 0):
                the unfused three-phase formula) and its live CUDA-event duration; `binding_unit` is the texture unit:
                filtered fetches per second achieved (live counters) over the ceiling measured in this process.
   cpu_baseline the single-thread C restatement (oracle/gipuma_oracle.c) on a FIXED band of rows of the N = 1 workload.
+--dump-outputs DIR writes what rank 0's last timed step computed (see dump_outputs); the inputs of a workload are the same
+in every run, so two builds can be compared output for output.
 --impl reference times the reference's own implementation of the path — gipuma.cu compiled unmodified for sm_100a
 (oracle/_ref, pins P1/P2 by macro, P3 for > 32 views) — on the same workload, same metric, on one GPU.  (The reference
 has no CPU implementation of this path; its CUDA kernels are "the reference's own implementation", DESIGN.md §7.)
@@ -55,6 +57,8 @@ sys.path.insert(0, ROOT)
 METRIC = "Mpixel-iters/s (ref-view PatchMatch sweep)"
 UNIT = "Mpixel-iters/s"
 FETCHES_PER_PAIR = 5          # bilinear fetches per (view, sample): centre, x+-1, y+-1 (gipuma.cu:251-253)
+DUMP_BYTES = 64 * 10 ** 6     # --dump-outputs: at most this much in all ...
+DUMP_PIXELS = 1 << 21         # ... else this many sampled pixels (20 B of outputs + 8 B of index each)
 
 
 class ClockSampler(threading.Thread):
@@ -167,6 +171,21 @@ def load_traffic(key):
         return t.get(key)
     except Exception:      # noqa: BLE001
         return None
+
+
+def dump_outputs(path, norm4, cost):
+    """The outputs of a run as the caller receives them: planes [H, W, 4] (world normal xyz, depth) as DIR/norm4.npy and
+    costs [H, W] as DIR/cost.npy, float32.  Above DUMP_BYTES the same fixed, seeded sample of DUMP_PIXELS pixels is
+    written for every run of the workload ([P, 4] and [P]), with their flat pixel indices as DIR/pixel_index.npy."""
+    os.makedirs(path, exist_ok=True)
+    norm4 = np.ascontiguousarray(norm4, dtype=np.float32)
+    cost = np.ascontiguousarray(cost, dtype=np.float32)
+    if norm4.nbytes + cost.nbytes > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(cost.size, DUMP_PIXELS, replace=False))
+        norm4, cost = norm4.reshape(-1, 4)[idx], cost.reshape(-1)[idx]
+        np.save(os.path.join(path, "pixel_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(path, "norm4.npy"), norm4)
+    np.save(os.path.join(path, "cost.npy"), cost)
 
 
 def cpu_baseline(sc, neighbours: int = 8) -> dict:
@@ -282,6 +301,7 @@ def run_ours_single_or_batch(args, mode, config, rank, world, local, sc):
         launches += st["launches"]
         pairs += st["pairs"];  hyp += st["hypotheses"];  skipped += st["skipped"];  pruned += st["pruned"]
     barrier()
+    outputs = ctx.get_state() if args.dump_outputs and rank == 0 else None    # the last timed step's result
     # ---- end to end through the public API, host buffers ------------------------------------------------------
     e2e_s = 0.0
     for _ in range(args.steps):
@@ -338,6 +358,8 @@ def run_ours_single_or_batch(args, mode, config, rank, world, local, sc):
         else:
             line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": 0, "kind": "port", "sample": "timed at N = 1 only"}
     ctx.close()
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, *outputs)
     return line
 
 
@@ -398,6 +420,7 @@ def run_ours_sharded(args, mode, config, shard, rank, world, local, sc):
         st = ctx.stats()
         launches += st["launches"];  collectives += st["collectives"];  pairs += st["pairs"];  hyp += st["hypotheses"];  skipped += st["skipped"]
     barrier()
+    outputs = ctx.get_state() if args.dump_outputs and rank == 0 else None    # group 0's result of the last timed step
     e2e_s = 0.0
     for _ in range(args.steps):
         flush.fill_(1)
@@ -465,6 +488,8 @@ def run_ours_sharded(args, mode, config, shard, rank, world, local, sc):
             "cpu_baseline": {"value": None, "unit": UNIT, "cores": 0, "kind": "port", "sample": "timed at N = 1 only"},
         }
     runner.close()
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, *outputs)
     return line
 
 
@@ -490,10 +515,12 @@ def run_reference(args, mode, config, shard, rank, world, local):
     sampler = ClockSampler(local)
 
     def run_once():
+        """(seconds of the reference's timed span, planes, costs)"""
         if args.neighbours == 20:                     # the kernels a reference built without SMALLKERNEL launches
-            _, _, ms = h.run_fused(sc)
-            return ms / 1e3
-        return h.run(sc)[2]
+            n4, c, ms = h.run_fused(sc)
+            return ms / 1e3, n4, c
+        n4, c, printed_s, _ = h.run(sc)
+        return printed_s, n4, c
 
     for _ in range(args.warmup):
         run_once()
@@ -501,10 +528,12 @@ def run_reference(args, mode, config, shard, rank, world, local):
     printed = wall = 0.0
     for _ in range(args.steps):
         t0 = time.perf_counter()
-        printed_s = run_once()
+        printed_s, n4, c = run_once()
         wall += time.perf_counter() - t0
         printed += printed_s
     clocks = sampler.finish()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, n4, c)
     units = args.steps * W * H * iters / 1e6
     value = units / printed
     return {
@@ -528,7 +557,7 @@ def run_reference(args, mode, config, shard, rank, world, local):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--mode", default="auto", choices=["auto", "single", "batch", "view_shard", "hybrid"])
@@ -542,7 +571,11 @@ def main():
     ap.add_argument("--color", action="store_true", help="float4 images (the reference's -color_processing)")
     ap.add_argument("--neighbours", type=int, default=8, choices=[8, 20],
                     help="20: the fused sweep of a reference built without SMALLKERNEL")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the planes and costs of the last timed step (rank 0's reference view) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     rank, world, local = dist_env()
     mode, config, shard = resolve(args, world)

@@ -114,6 +114,33 @@ def test_bench_arms_describe_the_same_workload():
             assert m == "view_shard" and cfg == 6 and shard == world
 
 
+def test_bench_dump_outputs_stays_within_64_mb_with_a_fixed_sample(tmp_path):
+    """bench.py --dump-outputs: whole outputs when they fit, else the same seeded pixel sample on every run."""
+    import importlib.util
+    import numpy as np
+    spec = importlib.util.spec_from_file_location("bench_module", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    rng = np.random.default_rng(3)
+    small = rng.standard_normal((120, 160, 4)).astype(np.float32), rng.standard_normal((120, 160)).astype(np.float32)
+    bench.dump_outputs(str(tmp_path / "small"), *small)
+    assert sorted(os.listdir(tmp_path / "small")) == ["cost.npy", "norm4.npy"]
+    assert np.array_equal(np.load(tmp_path / "small" / "norm4.npy"), small[0])
+    assert np.array_equal(np.load(tmp_path / "small" / "cost.npy"), small[1])
+    H, W = 2400, 3200                                         # BASELINE configs[4]: 154 MB of outputs
+    norm4 = np.broadcast_to(np.arange(H * W, dtype=np.float32).reshape(H, W, 1), (H, W, 4))
+    cost = -np.arange(H * W, dtype=np.float32).reshape(H, W)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), norm4, cost)
+        files = [tmp_path / run / f for f in ("norm4.npy", "cost.npy", "pixel_index.npy")]
+        assert sum(os.path.getsize(f) for f in files) <= 64 * 10 ** 6
+        idx = np.load(files[2])
+        assert idx.dtype == np.float64 and len(np.unique(idx)) == idx.size
+        assert np.array_equal(np.load(files[0])[:, 0], idx.astype(np.float32))
+        assert np.array_equal(np.load(files[1]), -idx.astype(np.float32))
+    assert np.array_equal(np.load(tmp_path / "a" / "pixel_index.npy"), np.load(tmp_path / "b" / "pixel_index.npy"))
+
+
 def test_batch_driver_validates_arguments_and_has_no_cpu_fallback():
     """gpm_batch_run (host C++): bad descriptors are refused before any CUDA call; without a device the workers fail loudly
     (no CPU path), with the reason in gpm_batch_last_error()."""

@@ -1,7 +1,7 @@
 """The reference's fused 20-neighbour sweep (gipuma_black_cu / gipuma_red_cu, gipuma.cu:1122-1351, 1714-1725, 1770-1781) —
 what `runcuda` launches when the reference is built without SMALLKERNEL (gipuma.cu:1913-1940) — selected here with
 gpm_set_option("neighbours", 20).  Bar: bit-exact, against committed golden outputs of the pinned reference build and
-against the live reference build when it travelled to the box."""
+against outputs of the reference build recorded on a B200 (oracle/recorded.py)."""
 import glob
 import os
 
@@ -19,13 +19,6 @@ def _load(name):
     from gipuma_b200.golden import scene_from_arrays
     z = dict(np.load(os.path.join(GOLDEN_DIR, name + ".npz")))
     return scene_from_arrays(name, z), z
-
-
-def _ref():
-    from oracle import pyref
-    if not os.path.exists(os.path.join(pyref.REF_DIR, "libhx_ref.so")):
-        pytest.skip("pinned reference build not present")
-    return pyref.Harness("ref")
 
 
 @pytest.mark.parametrize("name", FUSED)
@@ -70,23 +63,27 @@ LIVE = [
 
 
 @pytest.mark.parametrize("rows,cols,views,iters,box,nbest,comb,colour,seed", LIVE)
-def test_fused_full_run_bit_exact_vs_live_reference(rows, cols, views, iters, box, nbest, comb, colour, seed):
+def test_fused_full_run_bit_exact_vs_live_reference(request, rows, cols, views, iters, box, nbest, comb, colour, seed):
+    """Against the reference's outputs as recorded on a B200 (oracle/recorded.py)."""
     from gipuma_b200 import api, scene as S
-    from oracle import pyref
+    from oracle import recorded
     sc = S.make_config(4 if views > 10 else 2, rows=rows, cols=cols, n_views=views, iterations=iters, seed=3000 + seed)
     sc.params.box_hsize = sc.params.box_vsize = box
     sc.params.n_best = nbest
     sc.params.cost_comb = comb
     if colour:
         sc = S.colorize(sc)
-    which = "ref64" if views > 32 else "ref"
-    if not os.path.exists(os.path.join(pyref.REF_DIR, {"ref": "libhx_ref.so", "ref64": "libhx_ref64.so"}[which])):
-        pytest.skip("pinned reference build not present")
-    r_n4, r_c, _ = pyref.Harness(which).run_fused(sc, seed=seed)
+
+    def run():
+        from oracle import pyref
+        r_n4, r_c, _ = pyref.Harness("ref64" if views > 32 else "ref").run_fused(sc, seed=seed)
+        return {"norm4": r_n4, "cost": r_c}
+
+    ref = recorded.reference(request.node, run)
     for opts in ({}, {"memo": 0, "prune": 0, "dedupe": 0}):
         ls, _, _ = api.runcuda(sc, seed=seed, options=dict(opts, neighbours=20))
-        assert bits_equal(ls.norm4, r_n4) == 0
-        assert bits_equal(ls.c, r_c) == 0
+        assert ref.bits_differ("norm4", ls.norm4) == 0
+        assert ref.bits_differ("cost", ls.c) == 0
 
 
 def test_fused_mode_through_the_runcuda_adapter(monkeypatch):

@@ -1,22 +1,40 @@
-"""GPU parity against the LIVE pinned reference build (oracle/_ref/libhx_ref*.so), when it travelled to the box:
-fresh seeds, sizes and parameter corners that the committed golden fixtures do not cover."""
-import os
-
+"""GPU parity against the pinned reference build (oracle/_ref/libhx_ref*.so) on fresh seeds, sizes and parameter corners
+that the committed golden fixtures do not cover.  The reference's outputs are digests recorded on a B200
+(tests/golden/reference_outputs.json, oracle/recorded.py); GIPUMA_RECORD_REFERENCE records them again from the live build."""
 import numpy as np
 import pytest
 
-from conftest import bits_equal
+from oracle import recorded
 
 pytestmark = pytest.mark.gpu
 
 
 def _ref(n_views):
     from oracle import pyref
-    which = "ref64" if n_views > 32 else "ref"
-    path = os.path.join(pyref.REF_DIR, {"ref": "libhx_ref.so", "ref64": "libhx_ref64.so"}[which])
-    if not os.path.exists(path):
-        pytest.skip("pinned reference build not present")
-    return pyref.Harness(which)
+    return pyref.Harness("ref64" if n_views > 32 else "ref")
+
+
+def _run(sc, seed):
+    def run():
+        r_n4, r_c, printed_s, _ = _ref(sc.n_views).run(sc, seed=seed)
+        return {"norm4": r_n4, "cost": r_c, "printed_s": printed_s}
+    return run
+
+
+def _every_kernel(sc, seed):
+    """Init, the six kernels of one iteration (each from the reference's own previous state) and the final kernel."""
+    def run():
+        from oracle import pyref
+        ref = _ref(sc.n_views)
+        out = {}
+        n4, c, _ = ref.steps(sc, [pyref.STEP_INIT], seed=seed)
+        out["init_norm4"], out["init_cost"] = n4, c
+        for step in range(1, 7):
+            n4, c, _ = ref.steps(sc, [step], norm4=n4, cost=c, seed=seed)
+            out["step%d_norm4" % step], out["step%d_cost" % step] = n4, c
+        out["final_norm4"] = ref.steps(sc, [pyref.STEP_COMPUTE_DISP], norm4=n4, cost=c)[0]
+        return out
+    return run
 
 
 def reference_tile_fully_loaded(rows, cols, box):
@@ -50,18 +68,17 @@ CASES = [
 
 
 @pytest.mark.parametrize("cfg,rows,cols,views,iters,box,nbest,comb,seed", CASES)
-def test_full_run_bit_exact_vs_live_reference(cfg, rows, cols, views, iters, box, nbest, comb, seed):
+def test_full_run_bit_exact_vs_live_reference(request, cfg, rows, cols, views, iters, box, nbest, comb, seed):
     from gipuma_b200 import api, scene as S
     sc = S.make_config(cfg, rows=rows, cols=cols, n_views=views, iterations=iters, seed=1000 + seed)
     sc.params.box_hsize = sc.params.box_vsize = box
     sc.params.n_best = nbest
     sc.params.cost_comb = comb
     assert reference_tile_fully_loaded(rows, cols, box)
-    ref = _ref(sc.n_views)
-    r_n4, r_c, _, _ = ref.run(sc, seed=seed)
+    ref = recorded.reference(request.node, _run(sc, seed))
     ls, _, _ = api.runcuda(sc, seed=seed)
-    assert bits_equal(ls.norm4, r_n4) == 0
-    assert bits_equal(ls.c, r_c) == 0
+    assert ref.bits_differ("norm4", ls.norm4) == 0
+    assert ref.bits_differ("cost", ls.c) == 0
 
 
 COLOR_CASES = [
@@ -76,7 +93,7 @@ COLOR_CASES = [
 
 
 @pytest.mark.parametrize("rows,cols,views,iters,box,nbest,comb,seed", COLOR_CASES)
-def test_color_processing_full_run_bit_exact_vs_live_reference(rows, cols, views, iters, box, nbest, comb, seed):
+def test_color_processing_full_run_bit_exact_vs_live_reference(request, rows, cols, views, iters, box, nbest, comb, seed):
     """-color_processing: float4 images, runcuda<float4> (gipuma.cu:1965-1966)."""
     from gipuma_b200 import api, scene as S
     sc = S.colorize(S.make_config(4 if views > 10 else 2, rows=rows, cols=cols, n_views=views, iterations=iters,
@@ -85,38 +102,33 @@ def test_color_processing_full_run_bit_exact_vs_live_reference(rows, cols, views
     sc.params.n_best = nbest
     sc.params.cost_comb = comb
     assert reference_tile_fully_loaded(rows, cols, box)
-    ref = _ref(sc.n_views)
-    r_n4, r_c, _, _ = ref.run(sc, seed=seed)
+    ref = recorded.reference(request.node, _run(sc, seed))
     for opts in ({}, {"memo": 0, "prune": 0, "dedupe": 0}):
         ls, _, _ = api.runcuda(sc, seed=seed, options=opts)
-        assert bits_equal(ls.norm4, r_n4) == 0
-        assert bits_equal(ls.c, r_c) == 0
+        assert ref.bits_differ("norm4", ls.norm4) == 0
+        assert ref.bits_differ("cost", ls.c) == 0
 
 
-def test_color_every_kernel_of_one_iteration_vs_live_reference():
+def test_color_every_kernel_of_one_iteration_vs_live_reference(request):
     from gipuma_b200 import api, scene as S
-    from oracle import pyref
     sc = S.colorize(S.make_config(2, rows=96, cols=128, n_views=6, iterations=1, seed=4243))
     sc.params.box_hsize = sc.params.box_vsize = 13
-    ref = _ref(sc.n_views)
-    n4, c, _ = ref.steps(sc, [pyref.STEP_INIT], seed=99)
+    ref = recorded.reference(request.node, _every_kernel(sc, 99))
     with api.Context(sc.cols, sc.rows, sc.n_views) as ctx:
         ctx.load_scene(sc, seed=99)
         ctx.init()
         m4, mc = ctx.get_state()
-        assert bits_equal(m4, n4) == 0 and bits_equal(mc, c) == 0
+        assert ref.bits_differ("init_norm4", m4) == 0 and ref.bits_differ("init_cost", mc) == 0
         ctx.set_option("cost_variant", 3)                 # the initialisation kernel's rounding, on its own planes
-        assert bits_equal(ctx.cost_eval(n4), c) == 0
+        assert ref.bits_differ("init_cost", ctx.cost_eval(m4)) == 0
         for step, (colour, mask) in zip(range(1, 7), [(0, 1), (0, 2), (0, 4), (1, 1), (1, 2), (1, 4)]):
-            n4, c, _ = ref.steps(sc, [step], norm4=n4, cost=c, seed=99)
             ctx.phase(colour, mask)
             m4, mc = ctx.get_state()
-            assert bits_equal(m4, n4) == 0, "planes differ after reference kernel %d" % step
-            assert bits_equal(mc, c) == 0, "costs differ after reference kernel %d" % step
-        n4, c, _ = ref.steps(sc, [pyref.STEP_COMPUTE_DISP], norm4=n4, cost=c)
+            assert ref.bits_differ("step%d_norm4" % step, m4) == 0, "planes differ after reference kernel %d" % step
+            assert ref.bits_differ("step%d_cost" % step, mc) == 0, "costs differ after reference kernel %d" % step
         ctx.finalize()
         m4, mc = ctx.get_state()
-        assert bits_equal(m4, n4) == 0
+        assert ref.bits_differ("final_norm4", m4) == 0
 
 
 def test_color_and_gray_images_cannot_be_mixed():
@@ -130,85 +142,82 @@ def test_color_and_gray_images_cannot_be_mixed():
             ctx.set_view(0, np.ascontiguousarray(sc.images[1]), sc.cameras[1])
 
 
-def test_ragged_image_size_init_and_cost_bit_exact():
+def test_ragged_image_size_init_and_cost_bit_exact(request):
     """75 x 53 (no multiple of 32 or 16, narrower than two tiles).  The reference's sweep kernels read unloaded
     shared memory for such shapes, so only the stages that do not depend on its tile loader are compared:
     initialisation (texture path) and the cost function on identical planes (harness kernel, whole tile loaded)."""
     from gipuma_b200 import api, scene as S
-    from oracle import pyref
     sc = S.make_config(2, rows=53, cols=75, n_views=4, iterations=2, seed=77)
     sc.params.box_hsize = sc.params.box_vsize = 9
-    ref = _ref(sc.n_views)
-    n4, c, _ = ref.steps(sc, [pyref.STEP_INIT], seed=5)
-    rc = ref.cost_eval(sc, n4)
+
+    def run():
+        from oracle import pyref
+        ref = _ref(sc.n_views)
+        n4, c, _ = ref.steps(sc, [pyref.STEP_INIT], seed=5)
+        return {"init_norm4": n4, "init_cost": c, "sweep_cost": ref.cost_eval(sc, n4)}
+
+    ref = recorded.reference(request.node, run)
     with api.Context(sc.cols, sc.rows, sc.n_views) as ctx:
         ctx.load_scene(sc, seed=5)
         ctx.init()
         m4, mc = ctx.get_state()
-        assert bits_equal(m4, n4) == 0 and bits_equal(mc, c) == 0
-        assert bits_equal(ctx.cost_eval(n4), rc) == 0
+        assert ref.bits_differ("init_norm4", m4) == 0 and ref.bits_differ("init_cost", mc) == 0
+        assert ref.bits_differ("sweep_cost", ctx.cost_eval(m4)) == 0
         ctx.sweep(2)
         ctx.finalize()
         o4, oc = ctx.get_state()
     assert np.isfinite(o4).all() and np.isfinite(oc).all()
 
 
-def test_every_kernel_of_one_iteration_vs_live_reference():
+def test_every_kernel_of_one_iteration_vs_live_reference(request):
     from gipuma_b200 import api, scene as S
-    from oracle import pyref
     sc = S.make_config(2, rows=96, cols=128, n_views=7, iterations=1, seed=4242)
-    ref = _ref(sc.n_views)
-    n4, c, _ = ref.steps(sc, [pyref.STEP_INIT], seed=31337)
+    ref = recorded.reference(request.node, _every_kernel(sc, 31337))
     with api.Context(sc.cols, sc.rows, sc.n_views) as ctx:
         ctx.load_scene(sc, seed=31337)
         ctx.init()
         m4, mc = ctx.get_state()
-        assert bits_equal(m4, n4) == 0 and bits_equal(mc, c) == 0
+        assert ref.bits_differ("init_norm4", m4) == 0 and ref.bits_differ("init_cost", mc) == 0
         for step, (colour, mask) in zip(range(1, 7), [(0, 1), (0, 2), (0, 4), (1, 1), (1, 2), (1, 4)]):
-            n4, c, _ = ref.steps(sc, [step], norm4=n4, cost=c, seed=31337)
             ctx.phase(colour, mask)
             m4, mc = ctx.get_state()
-            assert bits_equal(m4, n4) == 0, "planes differ after reference kernel %d" % step
-            assert bits_equal(mc, c) == 0, "costs differ after reference kernel %d" % step
-        n4, c, _ = ref.steps(sc, [pyref.STEP_COMPUTE_DISP], norm4=n4, cost=c)
+            assert ref.bits_differ("step%d_norm4" % step, m4) == 0, "planes differ after reference kernel %d" % step
+            assert ref.bits_differ("step%d_cost" % step, mc) == 0, "costs differ after reference kernel %d" % step
         ctx.finalize()
         m4, mc = ctx.get_state()
-        assert bits_equal(m4, n4) == 0
+        assert ref.bits_differ("final_norm4", m4) == 0
 
 
-def test_non_8bit_images_stay_exact():
+def test_non_8bit_images_stay_exact(request):
     """Arbitrary (non-8-bit) float images."""
     from gipuma_b200 import api, scene as S
     sc = S.make_config(2, rows=96, cols=128, n_views=5, iterations=2, seed=2024)
     rng = np.random.default_rng(9)
     sc.images = (sc.images * 0.731 + rng.uniform(0, 3, size=sc.images.shape)).astype(np.float32)      # not integers
-    ref = _ref(sc.n_views)
-    r_n4, r_c, _, _ = ref.run(sc, seed=77)
+    ref = recorded.reference(request.node, _run(sc, 77))
     ls, _, _ = api.runcuda(sc, seed=77)
-    assert bits_equal(ls.norm4, r_n4) == 0 and bits_equal(ls.c, r_c) == 0
+    assert ref.bits_differ("norm4", ls.norm4) == 0 and ref.bits_differ("cost", ls.c) == 0
 
 
-def test_border_heavy_scene():
+def test_border_heavy_scene(request):
     """Small image, large window, strongly tilted random planes: many samples project onto or beyond the image border."""
     from gipuma_b200 import api, scene as S
     sc = S.make_config(2, rows=64, cols=64, n_views=4, iterations=3, seed=31)
     sc.params.box_hsize = sc.params.box_vsize = 21
-    ref = _ref(sc.n_views)
-    r_n4, r_c, _, _ = ref.run(sc, seed=123)
+    ref = recorded.reference(request.node, _run(sc, 123))
     for opts in ({}, {"memo": 0}):
         ls, _, _ = api.runcuda(sc, seed=123, options=opts)
-        assert bits_equal(ls.norm4, r_n4) == 0 and bits_equal(ls.c, r_c) == 0
+        assert ref.bits_differ("norm4", ls.norm4) == 0 and ref.bits_differ("cost", ls.c) == 0
 
 
-def test_baseline_config2_full_size_bit_exact_vs_live_reference():
+def test_baseline_config2_full_size_bit_exact_vs_live_reference(request):
     """BASELINE configs[1] as benchmarked: 1600 x 1200, 10 source views, 8 iterations, blocksize 15 — all 9.6 M output
     floats identical to the reference's."""
     from gipuma_b200 import api, scene as S
     sc = S.make_config(2)
     assert reference_tile_fully_loaded(sc.rows, sc.cols, sc.params.box_hsize)
-    ref = _ref(sc.n_views)
-    r_n4, r_c, printed_s, _ = ref.run(sc)
+    ref = recorded.reference(request.node, _run(sc, 0xC0FFEE))
     ls, ms, st = api.runcuda(sc)
-    assert bits_equal(ls.norm4, r_n4) == 0
-    assert bits_equal(ls.c, r_c) == 0
-    assert ms / 1e3 < printed_s          # and faster than the reference over the same span
+    assert ref.bits_differ("norm4", ls.norm4) == 0
+    assert ref.bits_differ("cost", ls.c) == 0
+    assert ms / 1e3 < ref["printed_s"]   # and faster than the reference over the same span (its time recorded on a B200)
